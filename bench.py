@@ -19,7 +19,7 @@ as sub-objects so that the driver's runs record them:
   N > 1 : batch32, tp_parity (TP-N vs TP1 logits on the workload's own weights, ids equal across ranks, tiny model vs
           the CPU oracle), llama2_70b (TP-N, with the TP1 anchor re-measured on rank 0), falcon_40b (N = 2, 4).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl b200|reference] [--no-extras]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl b200|reference] [--no-extras] [--dump-outputs DIR]
 """
 from __future__ import annotations
 
@@ -388,17 +388,20 @@ def measure(cx: Ctx, eng, vocab, B, steps, warmup, ttft_samples=TTFT_SAMPLES, co
     info = eng.info
     mx = cx.max_over_ranks if collective else (lambda v: v)
 
+    outputs = {}
+
     def one_request():
         sids = [eng.seq_create() for _ in range(B)]
         w0 = time.perf_counter()
         first, _ = eng.prefill(sids, prompts)  # host ids in (H2D inside), first token id back on the host
         w1 = time.perf_counter()
         pre_ms = eng.timing().prefill_ms
-        eng.decode(sids, first, NEW_TOKENS - 1)  # 127 device-resident steps, ids back on the host (D2H inside)
+        rest, _ = eng.decode(sids, first, NEW_TOKENS - 1)  # 127 device-resident steps, ids back on the host (D2H inside)
         w2 = time.perf_counter()
         dec_ms = eng.timing().decode_ms
         for s in sids:
             eng.seq_free(s)
+        outputs.update(prefill_tokens=first, decode_tokens=rest)  # the ids the caller receives; the top-up prefills below keep these
         return dict(ttft_wall_ms=(w1 - w0) * 1e3, prefill_dev_ms=pre_ms, decode_dev_ms=dec_ms,
                     decode_wall_ms=(w2 - w1) * 1e3, total_wall_ms=(w2 - w0) * 1e3)
 
@@ -449,7 +452,7 @@ def measure(cx: Ctx, eng, vocab, B, steps, warmup, ttft_samples=TTFT_SAMPLES, co
     return dict(value=steps * ntok / dec_dev_s, e2e=steps * ntok / dec_wall_s, wall=wall, clocks=clocks, tm=tm,
                 ttft_ms_p50=statistics.median(ttfts), prefill_device_ms_p50=statistics.median(pre_devs), ttft_samples=len(ttfts),
                 request_tok_s=steps * B * NEW_TOKENS / (sum(r["total_wall_ms"] for r in recs) / 1e3),
-                step_ms=step_ms, bytes_step=bytes_step, step_gbs=step_gbs, ctx_mean=ctx_mean)
+                step_ms=step_ms, bytes_step=bytes_step, step_gbs=step_gbs, ctx_mean=ctx_mean, outputs=outputs)
 
 
 def compact(cx: Ctx, m, B, load_s, eng, what):
@@ -676,7 +679,14 @@ def main():
     ap.add_argument("--graph", type=int, default=1)
     ap.add_argument("--engine-params", default="", help="JSON object merged into the engine's params.json (experiments, e.g. "
                     "'{\"tp_mega\": 1}'); echoed in config.engine_params so an overridden run is never mistaken for the default")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write the token ids the last timed request returned (prefill_tokens [B], "
+                         "decode_tokens [B, 127]) as float32 DIR/<name>.npy; inputs are seeded, so two builds compare id for id")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 path")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -708,6 +718,12 @@ def main():
 
     B = args.batch
     m = measure(cx, eng, cfg["vocab_size"], B, args.steps, args.warmup)
+    if args.dump_outputs and cx.rank == 0:
+        import numpy as np
+
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in m["outputs"].items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), np.asarray(a, dtype=np.float32))  # ids < 2^24: exact
     launches = int(m["tm"].kernel_launches)
     h2d, d2h = m["tm"].h2d_bytes // args.steps, m["tm"].d2h_bytes // args.steps
 

@@ -5,6 +5,7 @@ import os
 import subprocess
 import sys
 
+import pytest
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -49,10 +50,10 @@ def test_gpu_arm_refuses_without_a_gpu():
     assert r.returncode != 0 and "no CPU fallback" in (r.stderr + r.stdout)
 
 
-def test_gpu_arm_control_flow_against_a_mock_engine(monkeypatch, capsys):
+def test_gpu_arm_control_flow_against_a_mock_engine(monkeypatch, capsys, tmp_path):
     """bench.py's GPU arm end to end on CPU with a mock Engine (control flow and JSON contract, not numbers): the keys the
     driver reads, the TTFT top-up to >= 20 samples (SURVEY.md 8d), a failing batch-32 sub-measurement that must not lose
-    the headline line, --engine-params echoed in config."""
+    the headline line, --engine-params echoed in config, --dump-outputs writing the ids of the last timed request."""
     import importlib
     import time
 
@@ -68,7 +69,7 @@ def test_gpu_arm_control_flow_against_a_mock_engine(monkeypatch, capsys):
 
     class MockEngine:
         def __init__(self, model_dir, params):
-            self.info, self.params, self.n = Info(), params, 0
+            self.info, self.params, self.n, self.calls = Info(), params, 0, 0
 
         def seq_create(self):
             self.n += 1
@@ -81,11 +82,12 @@ def test_gpu_arm_control_flow_against_a_mock_engine(monkeypatch, capsys):
             if self.params.get("fail32") and len(sids) == 32:
                 raise RuntimeError("boom")
             time.sleep(0.001)
-            return np.zeros(len(sids), dtype=np.int32), None
+            self.calls += 1  # ids tell the requests apart
+            return np.full(len(sids), self.calls, dtype=np.int32), None
 
         def decode(self, sids, first, n):
             time.sleep(0.002)
-            return np.zeros((len(sids), n), dtype=np.int32), None
+            return np.tile(np.arange(n, dtype=np.int32), (len(sids), 1)) + first[:, None], None
 
         def timing(self):
             return Timing()
@@ -129,6 +131,15 @@ def test_gpu_arm_control_flow_against_a_mock_engine(monkeypatch, capsys):
     assert d["config"]["batch"] == 32 and "batch32" not in d and d["roofline"]["kernel"].startswith("gate/up")
     d = run(["--steps", "25", "--warmup", "1", "--no-cpu-baseline", "--no-batch32", "--no-extras"])
     assert d["ttft_samples"] == 25
+    out = tmp_path / "outputs"
+    run(["--steps", "3", "--warmup", "2", "--batch", "2", "--no-cpu-baseline", "--no-batch32", "--no-extras", "--dump-outputs", str(out)])
+    assert sorted(os.listdir(out)) == ["decode_tokens.npy", "prefill_tokens.npy"]
+    pre, dec = np.load(out / "prefill_tokens.npy"), np.load(out / "decode_tokens.npy")
+    assert pre.dtype == dec.dtype == np.float32 and pre.shape == (2,) and dec.shape == (2, bench.NEW_TOKENS - 1)
+    assert (pre == 5).all()  # prefill call 5 = the third timed request after two warm-ups, not a later TTFT top-up
+    assert (dec == 5 + np.arange(bench.NEW_TOKENS - 1)).all()
+    with pytest.raises(SystemExit):
+        run(["--steps", "0", "--no-cpu-baseline", "--no-extras"])
 
 
 def test_reference_arm_is_a_full_depth_measurement():
